@@ -1,6 +1,6 @@
 """bench.py -- dates x stocks / second per ELBO step (forward + backward [+ gradient all-reduce]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path (FactorVAE.forward + backward, reference module.py:250-270 +
@@ -45,7 +45,7 @@ WORKLOADS = {
 }
 C_FEATURES = 158
 METRIC = "dates x stocks / sec per ELBO step (fwd+bwd), K=20 C=158"
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 
 
 def f_fe(T, H, C=C_FEATURES):
@@ -72,8 +72,9 @@ def build_params(H, K, M, seed=42):
 
 
 def load_reference_module():
-    """The unmodified reference module.py from baseline/_ref (git-ignored copy staged by __graft_entry__.build()), or None."""
-    path = os.path.join(REF_DIR, "module.py")
+    """The unmodified reference module.py, byte-compiled into oracle/_ref by __graft_entry__.build() (oracle/stage_reference.py)
+    where the original project is present, or None."""
+    path = os.path.join(REF_DIR, "module.pyc")
     if not os.path.exists(path):
         return None
     spec = importlib.util.spec_from_file_location("fvae_reference_module", path)
@@ -201,8 +202,27 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(rows), "samples_under_load": len(busy)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, stepper, out):
+    """--dump-outputs: what a caller of the timed step holds after its last call, one float32 DIR/<name>.npy per array: the
+    global-batch loss and flat gradient (DateShardedStep.loss / .grad) and, when the step runs in one piece rather than in
+    micro-batches, the per-date and per-stock outputs of this rank's dates (the dict DateShardedStep.step returns)."""
+    import numpy as np
+    arrays = {"loss": stepper.loss, "grad": stepper.grad}
+    arrays.update((k, v) for k, v in (out or {}).items() if k != "loss")        # out["loss"] is stepper.loss
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_reference(args, wl, rank, world):
-    """Reference arm: the reference's own CPU implementation of the path -- the unmodified module.py from baseline/_ref
+    """Reference arm: the reference's own CPU implementation of the path -- the unmodified module.py from oracle/_ref
     (kind "reference"; oracle/cpu_port.py, kind "port", only if that copy is absent) -- on the host cores, one date per step as
     train_model.py does; each bench step = a bounded sample of `dates_per_step` dates of the workload's per-date shape."""
     if rank != 0:
@@ -223,7 +243,7 @@ def run_reference(args, wl, rank, world):
             st.train_step(x, y)
     dt = time.perf_counter() - t0
     value = args.steps * dates_per_step * wl["N"] / dt
-    what = "the unmodified reference module.py (baseline/_ref)" if st.kind == "reference" else "oracle/cpu_port.py (baseline/_ref absent)"
+    what = "the unmodified reference module.py (oracle/_ref)" if st.kind == "reference" else "oracle/cpu_port.py (oracle/_ref absent)"
     sample = (f"{dates_per_step} dates/step of the workload's per-date shape (N={wl['N']},T={wl['T']},K=H={wl['K']}), one date per "
               f"reference step (zero_grad, forward, loss.item(), backward; optimizer.step() not timed on either arm), fp32 torch CPU, "
               f"{what}, {cores} intra-op threads (fastest of 1..{ncpu} probed; host has {ncpu} CPUs)")
@@ -256,7 +276,7 @@ def time_eager_b200(wl, dev, budget_s=4.0):
     torch.cuda.synchronize()
     ms = (time.perf_counter() - t0) / n * 1e3
     return {"value": wl["N"] / (ms * 1e-3), "unit": "date*stocks/s", "ms_per_date": ms, "dates_timed": n,
-            "what": "unmodified reference module.py (baseline/_ref), PyTorch eager on this GPU, fp32, one date per step "
+            "what": "unmodified reference module.py (oracle/_ref), PyTorch eager on this GPU, fp32, one date per step "
                     "(zero_grad, forward, loss.item(), backward)"}
 
 
@@ -274,6 +294,7 @@ def main():
     ap.add_argument("--no-eager", action="store_true", help="skip the PyTorch-eager-on-B200 comparator")
     ap.add_argument("--collective", default="auto", choices=["auto", "p2p", "nccl"], help="gradient exchange: the one-kernel NVLink all-reduce or ncclAllReduce")
     ap.add_argument("--windows-e2e", action="store_true", help="also time the legacy variant that ships every window over PCIe")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -334,7 +355,7 @@ def main():
         date_ptr = engine.uniform_date_ptr(B, N, dev)
 
         def one_step():
-            stepper.step(x, y, date_ptr, global_dates=B_global, unit_base=unit_base, train=True)
+            return stepper.step(x, y, date_ptr, global_dates=B_global, unit_base=unit_base, train=True)[0]
     else:
         mbs = []
         for m0 in range(0, B, micro):
@@ -370,18 +391,23 @@ def main():
     for _ in range(int(extra.item())):
         one_step()
     barrier()
+    # the number of load steps above follows the clock: restart the Philox step counter so that the timed steps are always
+    # steps 1..K of the noise stream, and runs with the same arguments compute the same outputs
+    stepper.step_index = 0
     l0 = lib.fvae_debug_launch_count()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record()
     for _ in range(args.steps):
-        one_step()
+        last_out = one_step()
     ev1.record()
     barrier()
     launches = lib.fvae_debug_launch_count() - l0
     clocks = sampler.stop() if sampler else None
     ms = ev0.elapsed_time(ev1)
     loss_val = float(stepper.loss.item())
+    if args.dump_outputs and rank == 0:                 # before the sections below reuse the step's buffers
+        dump_outputs(args.dump_outputs, stepper, last_out)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -397,7 +423,7 @@ def main():
             for _ in range(max(3, args.warmup)):
                 g.replay()
             torch.cuda.synchronize()
-            nrep = max(50, args.steps)
+            nrep = args.steps
             g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             g0.record()
             for _ in range(nrep):
@@ -432,7 +458,7 @@ def main():
         out_k, st_k = engine.elbo_forward(layout, flat, xk, yk, engine.uniform_date_ptr(Sk // N, N, dev), train=True,
                                           precision="bf16", philox=(42, 1, unit_base))
         torch.cuda.synchronize()
-        reps = max(5, args.steps)
+        reps = args.steps
         for _ in range(3):
             engine.rerun_front_forward(st_k)
         k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -471,7 +497,7 @@ def main():
     # compute), fvae_window_index builds the look-back index, the ELBO kernels read the rows in place, the loss is copied to
     # pinned host memory and read there (the read of step i happens while step i+1 is queued: one-step-deferred logging).
     e2e = None
-    n_e2e = max(40, args.steps)
+    n_e2e = args.steps
     if not args.no_e2e and not strong:
         import numpy as np
         from factorvae_b200.panel import PanelIndex, ResidentPanel
@@ -603,7 +629,7 @@ def main():
     cpu_baseline = None
     if rank == 0 and not args.no_cpu_baseline:
         r = time_reference_cpu(wl, budget_s=10.0)
-        what = "the unmodified reference module.py (baseline/_ref)" if r["kind"] == "reference" else "oracle/cpu_port.py"
+        what = "the unmodified reference module.py (oracle/_ref)" if r["kind"] == "reference" else "oracle/cpu_port.py"
         cpu_baseline = {"value": r["value"], "unit": "date*stocks/s", "cores": r["cores"], "host_cpus": r["host_cpus"], "kind": r["kind"],
                         "sample": f"{r['steps']} per-date reference steps (N={N},T={T},K=H={K}; zero_grad, forward, loss.item(), backward; "
                                   f"no optimizer) in ~10 s, median {r['ms_per_date']:.2f} ms/date, fp32 torch CPU, {what}, "

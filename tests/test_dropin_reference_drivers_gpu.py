@@ -1,6 +1,6 @@
 """The drop-in proof (SURVEY section 4 item 4, section 8b): the reference's UNMODIFIED main.py / train_model.py / dataset.py /
-utils.py, taken from baseline/_ref (a git-ignored copy made by __graft_entry__.build() where /root/reference is mounted; it
-travels to the GPU box with the snapshot), import `module` from dropin/ and train on a synthetic (datetime, instrument) pickle:
+utils.py, byte-compiled into oracle/_ref by __graft_entry__.build() where the original project is present
+(oracle/stage_reference.py), import `module` from dropin/ and train on a synthetic (datetime, instrument) pickle:
 `from module import ...` (main.py:12, utils.py:6) resolves to the B200-native classes, main.main runs its epochs with Adam +
 CosineAnnealingLR on OUR parameters, writes its best-validation checkpoint, utils.load_model + load_state_dict reload it,
 train_model.validate and utils.generate_prediction_scores run on it.  The same harness is then run with the reference's own
@@ -15,7 +15,7 @@ import torch
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(ROOT, "oracle", "_ref")
 
 
 def _drive(module_dir, work, env_extra=None):
@@ -30,8 +30,8 @@ def _drive(module_dir, work, env_extra=None):
 
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
 def test_unmodified_reference_drivers_train_on_the_dropin(precision, tmp_path, cuda_device):
-    if not os.path.exists(os.path.join(REF, "main.py")):
-        pytest.skip("baseline/_ref is absent (built by __graft_entry__.build() where /root/reference is mounted)")
+    if not os.path.exists(os.path.join(REF, "main.pyc")):
+        pytest.skip("oracle/_ref is absent (made by __graft_entry__.build() where the original project is present)")
     ours = _drive(os.path.join(ROOT, "dropin"), tmp_path / "ours", {"FVAE_PRECISION": precision})
     print("drop-in driver result:", ours)
     assert ours["module_file"].startswith(os.path.join(ROOT, "dropin")), ours["module_file"]
